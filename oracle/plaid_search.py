@@ -7,8 +7,9 @@ What RA-VQA runs at evaluation time under DDP is ColBERT's PLAID pipeline on CPU
 (src/executors/FLMR_executor.py:778-792 -> colbert/searcher.py:91-132 -> IndexScorer.rank).  This
 module restates the Python glue of that pipeline and calls the reference's OWN native kernels,
 compiled in place by oracle/build_ref.py into oracle/_ref/ (filter_pids_cpp, decompress_residuals_cpp,
-segmented_lookup_cpp, segmented_maxsim_cpp).  A numpy restatement of filter_pids.cpp is kept beside
-it (filter_pids_np) so the pruning rule is spelled out and checked against the compiled kernel.
+segmented_lookup_cpp, segmented_maxsim_cpp).  Restatements of those four kernels are kept beside them
+(filter_pids_np, decompress_residuals_restated, segmented_lookup_restated, maxsim_oracle.segmented_maxsim)
+so the pruning rule is spelled out, and the search runs where the compiled kernels are absent.
 
 Pinned by tests/test_plaid_search.py against tests/golden/plaid_search.npz, which was produced by the
 reference's unmodified IndexScorer.rank / retrieve (tests/golden/make_golden_plaid_search.py).
@@ -35,7 +36,7 @@ import os
 import numpy as np
 import torch
 
-from . import build_ref
+from . import build_ref, maxsim_oracle
 
 _EXT = {}
 
@@ -215,12 +216,45 @@ class PlaidIndex:
 # ----------------------------------------------------------------------------------------------
 # search
 # ----------------------------------------------------------------------------------------------
-def decompress(index: PlaidIndex, pids: torch.Tensor) -> torch.Tensor:
-    """index_storage.py:160-173: decompress_residuals_cpp over `pids` (int32), then fp32 L2 normalise."""
-    D = _ext("decompress_residuals_cpp").decompress_residuals_cpp(
-        pids, index.doclens, index.offsets, index.bucket_weights, index.reversed_bit_map, index.lut,
-        index.residuals, index.codes, index.centroids, index.dim, index.nbits)
+def decompress(index: PlaidIndex, pids: torch.Tensor, compiled: bool | None = None) -> torch.Tensor:
+    """index_storage.py:160-173: decompress_residuals_cpp over `pids` (int32), then fp32 L2 normalise.
+
+    `compiled`: use the reference's compiled kernel (True) or decompress_residuals_restated (False);
+    None = the compiled kernel when oracle/_ref holds it."""
+    if compiled is None:
+        compiled = have_reference_kernels()
+    if compiled:
+        D = _ext("decompress_residuals_cpp").decompress_residuals_cpp(
+            pids, index.doclens, index.offsets, index.bucket_weights, index.reversed_bit_map, index.lut,
+            index.residuals, index.codes, index.centroids, index.dim, index.nbits)
+    else:
+        D = decompress_residuals_restated(index, pids)
     return torch.nn.functional.normalize(D.to(torch.float32), p=2, dim=-1)
+
+
+def _token_rows(index: PlaidIndex, pids: torch.Tensor) -> torch.Tensor:
+    """Embedding ids of the passages `pids`, passage by passage, in token order."""
+    pids = pids.long()
+    lengths = index.doclens[pids]
+    starts = torch.repeat_interleave(index.offsets[pids], lengths)
+    first = torch.repeat_interleave(torch.cumsum(lengths, 0) - lengths, lengths)
+    return starts + torch.arange(int(lengths.sum())) - first
+
+
+def decompress_residuals_restated(index: PlaidIndex, pids: torch.Tensor) -> torch.Tensor:
+    """torch restatement of search/decompress_residuals.cpp: for every token of every passage in `pids`,
+    each residual byte goes through reversed_bit_map, then the lookup table gives its 8/nbits bucket
+    indices; output[t, d] = bucket_weights[bucket index of d] + centroids[code of t, d] (fp32, unnormalised)."""
+    rows = _token_rows(index, pids)
+    buckets = index.lut[index.reversed_bit_map[index.residuals[rows].long()].long()].reshape(rows.numel(), index.dim)
+    return index.bucket_weights[buckets.long()] + index.centroids[index.codes[rows].long()]
+
+
+def segmented_lookup_restated(ivf, cells, lengths, offsets) -> torch.Tensor:
+    """torch restatement of search/segmented_lookup.cpp: ivf[offsets[i] : offsets[i] + lengths[i]] of every
+    cell, concatenated in cell order."""
+    return torch.cat([ivf[int(o): int(o) + int(n)] for o, n in zip(offsets.tolist(), lengths.tolist())]
+                     + [ivf[:0]])
 
 
 def filter_pids_np(pids, centroid_scores, codes, doclens, offsets, idx, ndocs):
@@ -256,10 +290,12 @@ def filter_pids_np(pids, centroid_scores, codes, doclens, offsets, idx, ndocs):
 
 
 class PlaidSearcher:
-    """IndexScorer (CPU, `use_gpu=False`) over a PlaidIndex, built on the reference's compiled kernels."""
+    """IndexScorer (CPU, `use_gpu=False`) over a PlaidIndex, built on the reference's compiled kernels, or on
+    their restatements in this module where oracle/_ref does not hold them (`compiled` says which)."""
 
-    def __init__(self, index: PlaidIndex):
+    def __init__(self, index: PlaidIndex, compiled: bool | None = None):
         self.index = index
+        self.compiled = have_reference_kernels() if compiled is None else bool(compiled)
 
     def get_cells(self, Q, ncells):
         """candidate_generation.py:11-20.  Q [nq,128] fp32 -> (unique cell ids, centroid scores [K,nq])."""
@@ -280,8 +316,9 @@ class PlaidSearcher:
         assert Qc.dim() == 2
         cells, centroid_scores = self.get_cells(Qc, ncells)
         cells = cells.long()
-        pids = _ext("segmented_lookup_cpp").segmented_lookup_cpp(
-            ix.ivf, cells, ix.ivf_lengths[cells], ix.ivf_offsets[cells])
+        lookup = (_ext("segmented_lookup_cpp").segmented_lookup_cpp if self.compiled
+                  else segmented_lookup_restated)
+        pids = lookup(ix.ivf, cells, ix.ivf_lengths[cells], ix.ivf_offsets[cells])
         pids = torch.unique_consecutive(pids.sort().values)
         return pids, centroid_scores
 
@@ -289,12 +326,18 @@ class PlaidSearcher:
         """index_storage.py:102-182, CPU branch, Q.size(0) == 1."""
         ix = self.index
         idx = centroid_scores.max(-1).values >= threshold                                        # :114
-        pids = _ext("filter_pids_cpp").filter_pids_cpp(pids, centroid_scores, ix.codes, ix.doclens, ix.offsets,
-                                                       idx, ndocs)                              # :153-156
-        D_packed = decompress(ix, pids)                                                          # :160-173
+        if self.compiled:
+            pids = _ext("filter_pids_cpp").filter_pids_cpp(pids, centroid_scores, ix.codes, ix.doclens,
+                                                           ix.offsets, idx, ndocs)              # :153-156
+        else:
+            pids = torch.from_numpy(filter_pids_np(pids.numpy(), centroid_scores.numpy(), ix.codes.numpy(),
+                                                   ix.doclens.numpy(), ix.offsets.numpy(), idx.numpy(), ndocs))
+        D_packed = decompress(ix, pids, self.compiled)                                           # :160-173
         D_lengths = ix.doclens[pids.long()]                                                      # :174
         scores = D_packed @ Q.squeeze(0).to(dtype=D_packed.dtype).T                              # colbert.py:303-305
-        return _ext("segmented_maxsim_cpp").segmented_maxsim_cpp(scores, D_lengths), pids       # colbert.py:311
+        if self.compiled:
+            return _ext("segmented_maxsim_cpp").segmented_maxsim_cpp(scores, D_lengths), pids   # colbert.py:311
+        return torch.from_numpy(maxsim_oracle.segmented_maxsim(scores.numpy(), D_lengths.numpy())), pids
 
     def rank(self, Q, ncells=2, threshold=0.45, ndocs=1024, query_maxlen=32):
         """IndexScorer.rank (index_storage.py:86-100) for one query Q [1,Nq,128] fp32 -> (pids, scores) lists.

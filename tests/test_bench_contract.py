@@ -39,17 +39,16 @@ def test_reference_arm_other_ranks_exit_quietly():
 
 
 def test_plaid_cpu_baseline_leg_runs_on_a_small_sample():
-    """bench.py's PLAID leg (restated IndexScorer.rank over the reference's compiled kernels), CPU build."""
+    """bench.py's PLAID leg (restated IndexScorer.rank over the reference's compiled kernels where they were
+    built, else over their restatements), CPU build."""
     import types
 
-    import pytest
     sys.path.insert(0, ROOT)
     import bench
     from oracle import plaid_search as P
-    if not P.have_reference_kernels():
-        pytest.skip("oracle/_ref/*.so not built")
     args = types.SimpleNamespace(plaid_passages=1000, nd=60, nq=64, k=5, plaid_ndocs=16)
     out = bench.cpu_plaid_rate(args, "cpu", target_seconds=1.0)
-    assert out["kind"] == "reference" and out["value"] > 0 and out["cores"] >= 1
+    assert out["kind"] == ("reference" if P.have_reference_kernels() else "port")
+    assert out["value"] > 0 and out["cores"] >= 1
     assert out["recall_at_5"] >= 0.9          # clustered data: PLAID finds the planted passage
     assert min(out["candidates_per_query"]) >= 16 and "NOT extrapolated" in out["sample"]

@@ -1,6 +1,6 @@
 """CPU: pin the oracle (numpy + C restatements) against golden vectors produced by the reference's
-own code (tests/golden/make_golden.py), and against the reference's compiled segmented_maxsim.cpp
-(oracle/_ref) when it is present."""
+own code (tests/golden/make_golden.py, make_golden_reference_checks.py), and against the reference's compiled
+segmented_maxsim.cpp (oracle/_ref) when it is present."""
 import os
 import sys
 
@@ -99,18 +99,20 @@ def test_bf16_round_matches_torch():
 
 
 def test_reference_extension_agrees_when_present():
-    """oracle/_ref/segmented_maxsim_cpp.so is the REFERENCE's own segmented_maxsim.cpp (build_ref.py)."""
+    """O.segmented_maxsim against what the REFERENCE's own segmented_maxsim.cpp returned
+    (tests/golden/make_golden_reference_checks.py), and against the compiled extension itself where
+    oracle/build_ref.py built it into oracle/_ref/."""
+    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+    import make_golden_reference_checks as G
+    z = np.load(os.path.join(ROOT, "tests", "golden", "reference_checks.npz"))
+    scores, lengths = G.segmented_inputs()
+    got = O.segmented_maxsim(scores.numpy(), lengths.numpy())
+    np.testing.assert_allclose(got, z["segmented_maxsim"], rtol=1e-6, atol=1e-5)
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import build_ref
     mod = build_ref.load()
-    if mod is None:
-        pytest.skip("oracle/_ref/segmented_maxsim_cpp.so not built (needs /root/reference)")
-    import torch
-    rng = np.random.default_rng(1)
-    lengths = rng.integers(1, 40, size=50)
-    scores = rng.standard_normal((int(lengths.sum()), 33)).astype(np.float32)
-    ref = mod.segmented_maxsim_cpp(torch.from_numpy(scores), torch.from_numpy(lengths).long()).numpy()
-    np.testing.assert_allclose(O.segmented_maxsim(scores, lengths), ref, rtol=1e-6, atol=1e-5)
+    if mod is not None:
+        np.testing.assert_allclose(got, mod.segmented_maxsim_cpp(scores, lengths).numpy(), rtol=1e-6, atol=1e-5)
 
 
 def test_training_path_restatement_matches_reference_autograd():

@@ -2,10 +2,10 @@
 
 tests/golden/plaid_search.npz holds what the unmodified reference returned (candidate pids, centroid
 scores, pids surviving filter_pids.cpp, final ranking) — see tests/golden/make_golden_plaid_search.py.
-The search tests need the reference's native kernels compiled into oracle/_ref/ (oracle/build_ref.py,
-run by __graft_entry__.build() in the build container); the pruning rule is also checked through the
-numpy restatement, which needs nothing.
+The search tests run the oracle on its restatements of the reference's native kernels and, where
+oracle/build_ref.py compiled them into oracle/_ref/, on the compiled kernels as well.
 """
+import itertools
 import os
 
 import numpy as np
@@ -15,8 +15,11 @@ import torch
 from oracle import plaid_search as P
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "plaid_search.npz")
-needs_ref = pytest.mark.skipif(not P.have_reference_kernels(),
-                               reason="oracle/_ref/*.so not built (python oracle/build_ref.py)")
+
+
+def _searchers(index):
+    """The restated kernels always; the reference's compiled kernels too where they were built."""
+    return [P.PlaidSearcher(index, compiled=c) for c in ([False, True] if P.have_reference_kernels() else [False])]
 
 
 @pytest.fixture(scope="module")
@@ -76,11 +79,9 @@ def test_filter_pids_restatement_rejects_undefined_case(index):
                          np.ones(cs.shape[0], dtype=bool), 8)
 
 
-@needs_ref
 def test_retrieve_matches_reference(gold, index):
-    s = P.PlaidSearcher(index)
     Q = torch.from_numpy(gold["queries"])
-    for ci, (ncells, thr, ndocs, qmax) in enumerate(_configs(gold)):
+    for s, (ci, (ncells, thr, ndocs, qmax)) in itertools.product(_searchers(index), enumerate(_configs(gold))):
         for qi in range(Q.size(0)):
             key = "c%d_q%d_" % (ci, qi)
             cand, cs = s.retrieve(Q[qi:qi + 1], ncells, qmax)
@@ -88,11 +89,9 @@ def test_retrieve_matches_reference(gold, index):
             np.testing.assert_allclose(cs.numpy(), gold[key + "cscores"], rtol=0, atol=1e-6)
 
 
-@needs_ref
 def test_rank_matches_reference(gold, index):
-    s = P.PlaidSearcher(index)
     Q = torch.from_numpy(gold["queries"])
-    for ci, (ncells, thr, ndocs, qmax) in enumerate(_configs(gold)):
+    for s, (ci, (ncells, thr, ndocs, qmax)) in itertools.product(_searchers(index), enumerate(_configs(gold))):
         for qi in range(Q.size(0)):
             key = "c%d_q%d_" % (ci, qi)
             pids, scores = s.rank(Q[qi:qi + 1], ncells=ncells, threshold=thr, ndocs=ndocs, query_maxlen=qmax)
@@ -101,17 +100,16 @@ def test_rank_matches_reference(gold, index):
             assert len(pids) == ndocs // 4
 
 
-@needs_ref
 def test_rank_is_a_subset_of_exhaustive_scoring(gold, index):
     """PLAID's final scores are exact MaxSim over the DEcompressed index, on a pruned passage set."""
     from oracle import maxsim_oracle as O
-    D = index.decompress_all().numpy()
     Q = gold["queries"]
-    exact = O.maxsim_scores(Q, D, index.doclens.numpy().astype(np.int32), relu=True)
-    s = P.PlaidSearcher(index)
     ncells, thr, ndocs, qmax = _configs(gold)[2]
-    for qi in range(Q.shape[0]):
-        pids, scores = s.rank(torch.from_numpy(Q[qi:qi + 1]), ncells=ncells, threshold=thr, ndocs=ndocs,
-                              query_maxlen=qmax)
-        np.testing.assert_allclose(exact[qi, pids], scores, rtol=2e-6, atol=2e-6)
-        assert scores[0] <= exact[qi].max() + 1e-5
+    for s in _searchers(index):
+        D = P.decompress(index, torch.arange(index.doclens.numel(), dtype=torch.int32), s.compiled).numpy()
+        exact = O.maxsim_scores(Q, D, index.doclens.numpy().astype(np.int32), relu=True)
+        for qi in range(Q.shape[0]):
+            pids, scores = s.rank(torch.from_numpy(Q[qi:qi + 1]), ncells=ncells, threshold=thr, ndocs=ndocs,
+                                  query_maxlen=qmax)
+            np.testing.assert_allclose(exact[qi, pids], scores, rtol=2e-6, atol=2e-6)
+            assert scores[0] <= exact[qi].max() + 1e-5

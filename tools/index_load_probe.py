@@ -1,5 +1,5 @@
 """Index-load throughput (GPU box): write a synthetic flat index of `--gigabytes` to `--dir` (chunks of 25k
-passages, as the Indexer writes them), drop it from the page cache if allowed, and time FlatCorpus.from_index —
+passages, as the Indexer writes them), evict its files from the page cache, and time FlatCorpus.from_index —
 the C-level streaming builder (pread into two pinned buffers with 8 threads, overlapped H2D, padded layout).
 
     python tools/index_load_probe.py --gigabytes 8 --dir /dev/shm/flmr_idx
@@ -42,13 +42,18 @@ def main():
     t_write = time.perf_counter() - t0
     size = sum(os.path.getsize(os.path.join(args.dir, f)) for f in os.listdir(args.dir)) / 1e9
     print("wrote %.2f GB in %d chunks to %s (%.1f s)" % (size, c, args.dir, t_write), flush=True)
+    # evict only this index's own pages (a per-file hint; clean pages of these files are dropped)
     cold = False
     try:
-        os.sync()
-        with open("/proc/sys/vm/drop_caches", "w") as f:
-            f.write("1\n")
+        for f in os.listdir(args.dir):
+            fd = os.open(os.path.join(args.dir, f), os.O_RDONLY)
+            try:
+                os.fsync(fd)
+                os.posix_fadvise(fd, 0, 0, os.POSIX_FADV_DONTNEED)
+            finally:
+                os.close(fd)
         cold = True
-    except Exception:
+    except (OSError, AttributeError):
         pass
     for attempt in ("cold" if cold else "page-cache", "page-cache"):
         torch.cuda.synchronize()
