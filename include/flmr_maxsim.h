@@ -76,6 +76,7 @@ typedef struct flmr_corpus flmr_corpus_t;       /* resident passage-token shard 
 typedef struct flmr_workspace flmr_workspace_t; /* per-caller scratch (candidates, Q pad)  */
 typedef struct flmr_comm flmr_comm_t;           /* this rank's end of the shard exchange   */
 typedef struct flmr_corpus_builder flmr_corpus_builder_t; /* streaming index load          */
+typedef struct flmr_corpus_plaid_builder flmr_corpus_plaid_builder_t; /* chunked compressed load */
 
 typedef struct flmr_corpus_info {
   int64_t n_passages;     /* passages in this shard                                           */
@@ -88,6 +89,7 @@ typedef struct flmr_corpus_info {
   int32_t adopted;        /* 1 if the token matrix is the caller's buffer (zero-copy)         */
   int64_t n_tiles;        /* passage-token tiles streamed per corpus pass                     */
   int64_t hbm_bytes;      /* bytes of HBM held by the handle (excluding an adopted matrix)    */
+                          /* (flmr_corpus_create_plaid: the compressed arrays + centroids)    */
 } flmr_corpus_info_t;
 
 /* Thread-local description of the last error returned on this thread ("" if none). */
@@ -107,6 +109,38 @@ int flmr_abi_version(void);
  */
 int flmr_corpus_create(const void* tokens, const int32_t* h_doclens, int64_t n_passages, int dim,
                        int device, int64_t pid_base, unsigned flags, flmr_corpus_t** out);
+/*
+ * Create a resident corpus shard that stays COMPRESSED in HBM: the PLAID (ColBERTv2 residual) arrays of an index
+ * written by the reference's Indexer, decoded inside the scan kernel instead of once into bf16 (flmr_plaid_decode).
+ * Searches return exactly what a corpus created from the decoded tokens returns; the shard takes
+ * 4 (code) + 16 * nbits (residual) + 4 (inverse norm) bytes per stored row instead of 256.
+ *   d_codes          int32 [sum(h_doclens)]                    (<c>.codes.pt, passage after passage)
+ *   d_residuals      uint8 [sum(h_doclens), dim * nbits / 8]   (<c>.residuals.pt)
+ *   d_centroids      fp32  [n_centroids, dim]                  (centroids.pt, upcast; copied)
+ *   d_bucket_weights fp32  [2^nbits]                            (buckets.pt[1]; copied)
+ *   nbits            1, 2, 4 or 8;  h_doclens / pid_base as flmr_corpus_create
+ * All d_ arrays are device pointers on `device` and may be freed when the call returns.  Every code is checked
+ * against [0, n_centroids) here (FLMR_ERR_INVALID_ARG otherwise), never during a search.  Every entry point taking
+ * a corpus accepts the handle; flmr_debug_maxsim_scores_simt returns FLMR_ERR_UNSUPPORTED for it.  Synchronous.
+ */
+int flmr_corpus_create_plaid(const int32_t* d_codes, const uint8_t* d_residuals, const float* d_centroids,
+                             int64_t n_centroids, const float* d_bucket_weights, int nbits, const int32_t* h_doclens,
+                             int64_t n_passages, int dim, int device, int64_t pid_base, flmr_corpus_t** out);
+/*
+ * The same, chunk by chunk — the load path of a large index: builder_create allocates the handle's arrays from the
+ * doclens (and copies the centroids and bucket weights), every append packs the next chunk of WHOLE passages
+ * (d_codes int32 [n_tokens], d_residuals uint8 [n_tokens, dim * nbits / 8], device pointers, passage after passage
+ * in order; synchronous, the chunk may be freed on return), finish checks the codes of every chunk and hands over
+ * the corpus (the builder is destroyed).  Peak device memory of a load = the resident arrays + one chunk.
+ * A shard holds fewer than 2^31 - FLMR_TILE_TOKENS stored rows (as every corpus handle).
+ */
+int flmr_corpus_plaid_builder_create(const float* d_centroids, int64_t n_centroids, const float* d_bucket_weights,
+                                     int nbits, const int32_t* h_doclens, int64_t n_passages, int dim, int device,
+                                     int64_t pid_base, flmr_corpus_plaid_builder_t** out);
+int flmr_corpus_plaid_builder_append(flmr_corpus_plaid_builder_t* b, const int32_t* d_codes,
+                                     const uint8_t* d_residuals, int64_t n_tokens);
+int flmr_corpus_plaid_builder_finish(flmr_corpus_plaid_builder_t* b, flmr_corpus_t** out);
+int flmr_corpus_plaid_builder_destroy(flmr_corpus_plaid_builder_t* b);
 int flmr_corpus_destroy(flmr_corpus_t* corpus);
 int flmr_corpus_info(const flmr_corpus_t* corpus, flmr_corpus_info_t* out);
 

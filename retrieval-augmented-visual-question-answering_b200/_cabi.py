@@ -33,7 +33,9 @@ TILE_TOKENS = _header_define("FLMR_TILE_TOKENS")
 # every symbol include/flmr_maxsim.h declares (tests check the .so exports all of them)
 SYMBOLS = [
     "flmr_last_error", "flmr_abi_version",
-    "flmr_corpus_create", "flmr_corpus_destroy", "flmr_corpus_info",
+    "flmr_corpus_create", "flmr_corpus_create_plaid", "flmr_corpus_destroy",
+    "flmr_corpus_plaid_builder_create", "flmr_corpus_plaid_builder_append", "flmr_corpus_plaid_builder_finish",
+    "flmr_corpus_plaid_builder_destroy", "flmr_corpus_info",
     "flmr_workspace_create", "flmr_workspace_destroy", "flmr_workspace_status",
     "flmr_maxsim_scores", "flmr_maxsim_topk", "flmr_topk_merge", "flmr_topk_select", "flmr_plaid_decode",
     "flmr_maxsim_argmax", "flmr_maxsim_backward", "flmr_corpus_gather",
@@ -78,6 +80,11 @@ def lib() -> C.CDLL:
     L.flmr_abi_version.restype = i32
     L.flmr_abi_version.argtypes = []
     L.flmr_corpus_create.argtypes = [vp, vp, i64, i32, i32, i64, u32, C.POINTER(vp)]
+    L.flmr_corpus_create_plaid.argtypes = [vp, vp, vp, i64, vp, i32, vp, i64, i32, i32, i64, C.POINTER(vp)]
+    L.flmr_corpus_plaid_builder_create.argtypes = [vp, i64, vp, i32, vp, i64, i32, i32, i64, C.POINTER(vp)]
+    L.flmr_corpus_plaid_builder_append.argtypes = [vp, vp, vp, i64]
+    L.flmr_corpus_plaid_builder_finish.argtypes = [vp, C.POINTER(vp)]
+    L.flmr_corpus_plaid_builder_destroy.argtypes = [vp]
     L.flmr_corpus_destroy.argtypes = [vp]
     L.flmr_corpus_info.argtypes = [vp, C.POINTER(CorpusInfo)]
     L.flmr_workspace_create.argtypes = [vp, i32, i32, C.POINTER(vp)]

@@ -75,9 +75,11 @@ class FlatCorpus:
         self._ws = None
         self.pid_base = int(pid_base)
         self.load_stats = None
+        self.nbits = 0
 
     @classmethod
-    def _from_handle(cls, handle, doclens: np.ndarray, device: torch.device, pid_base: int) -> "FlatCorpus":
+    def _from_handle(cls, handle, doclens: np.ndarray, device: torch.device, pid_base: int,
+                     nbits: int = 0) -> "FlatCorpus":
         self = cls.__new__(cls)
         self.doclens = doclens
         self.device = device
@@ -89,6 +91,7 @@ class FlatCorpus:
         self._ws = None
         self.pid_base = int(pid_base)
         self.load_stats = None
+        self.nbits = int(nbits)      # != 0: the handle came from flmr_corpus_create_plaid / the PLAID builder
         return self
 
     @classmethod
@@ -143,19 +146,39 @@ class FlatCorpus:
 
     @classmethod
     def from_plaid(cls, path: str, device=None, rank: int = 0, world_size: int = 1) -> "FlatCorpus":
-        """Decode a reference PLAID index directory on the GPU (plaid.py) and keep it resident — with
-        world_size > 1 only this rank's contiguous, token-balanced passage shard (SURVEY.md 8e)."""
-        from .plaid import plaid_to_flat, read_plaid_doclens, read_plaid_metadata
+        """Load a reference PLAID index directory (plaid.py) and keep it resident — with world_size > 1 only
+        this rank's contiguous, token-balanced passage shard (SURVEY.md 8e).  The shard is decoded into bf16 on
+        the GPU when that fits the device's free memory (plaid.keep_compressed); otherwise it stays compressed in
+        HBM and the scan decodes it on the fly.  Either way searches return the same bits."""
+        from .plaid import plaid_to_compressed, plaid_to_flat, read_plaid_doclens, read_plaid_metadata, use_compressed
         from .sharded import shard_ranges
-        if world_size == 1:
-            tokens, doclens = plaid_to_flat(path, device)
-            return cls(tokens, doclens, device=tokens.device)
+        if not torch.cuda.is_available():
+            raise RuntimeError("FlatCorpus needs a CUDA device: there is no CPU fallback for this path")
         all_doclens = np.concatenate(read_plaid_doclens(path, read_plaid_metadata(path)["num_chunks"]))
-        p0, p1 = shard_ranges(all_doclens, world_size)[rank]
+        p0, p1 = shard_ranges(all_doclens, world_size)[rank] if world_size > 1 else (0, len(all_doclens))
         if p0 == p1:
             return None
-        tokens, doclens = plaid_to_flat(path, device, passage_range=(p0, p1))
+        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        if dev.index is None:
+            dev = torch.device("cuda", torch.cuda.current_device())
+        if use_compressed(all_doclens[p0:p1], dev):
+            handle, doclens, nbits = plaid_to_compressed(path, dev, passage_range=(p0, p1))
+            return cls._from_handle(handle, doclens, dev, p0, nbits=nbits)
+        tokens, doclens = plaid_to_flat(path, dev, passage_range=(p0, p1))
         return cls(tokens, doclens, device=tokens.device, pid_base=p0)
+
+    @classmethod
+    def from_plaid_arrays(cls, codes: torch.Tensor, residuals: torch.Tensor, centroids: torch.Tensor,
+                          bucket_weights: torch.Tensor, nbits: int, doclens, device=None, pid_base: int = 0,
+                          chunk_passages: Optional[int] = None) -> "FlatCorpus":
+        """A compressed shard from PLAID arrays already on the GPU (codes int32, residuals uint8, centroids and
+        bucket weights fp32; see plaid.create_compressed)."""
+        from .plaid import create_compressed
+        dev = codes.device if device is None else torch.device(device)
+        dl = _as_doclens(doclens)
+        handle = create_compressed(codes, residuals, centroids, bucket_weights, nbits, dl, dev, pid_base,
+                                   chunk_passages=chunk_passages)
+        return cls._from_handle(handle, dl, dev, pid_base, nbits=nbits)
 
     # -- properties ---------------------------------------------------------------------------
     @property
@@ -165,6 +188,11 @@ class FlatCorpus:
     @property
     def n_tokens(self) -> int:
         return int(self.info.n_tokens)
+
+    @property
+    def compressed(self) -> bool:
+        """True when the shard is held as PLAID codes + residuals (``nbits`` per dim) and decoded by the scan."""
+        return self.nbits != 0
 
     @property
     def handle(self) -> C.c_void_p:
@@ -217,5 +245,5 @@ class FlatCorpus:
 
     def __repr__(self) -> str:
         i = self.info
-        return ("FlatCorpus(n_passages=%d, n_tokens=%d, device=%s, pid_base=%d, n_ctas=%d, adopted=%d)"
-                % (i.n_passages, i.n_tokens, self.device, i.pid_base, i.n_ctas, i.adopted))
+        return ("FlatCorpus(n_passages=%d, n_tokens=%d, device=%s, pid_base=%d, n_ctas=%d, adopted=%d, nbits=%d)"
+                % (i.n_passages, i.n_tokens, self.device, i.pid_base, i.n_ctas, i.adopted, self.nbits))

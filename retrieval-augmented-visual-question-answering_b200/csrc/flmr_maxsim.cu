@@ -19,6 +19,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <limits>
 #include <mutex>
 #include <new>
@@ -30,6 +31,7 @@
 
 #include "../../include/flmr_maxsim.h"
 #include "flmr_scan_kernel.cuh"
+#include "flmr_scan_plaid_kernel.cuh"
 #include "flmr_scan3_kernel.cuh"
 #include "flmr_train_kernels.cuh"
 #include "flmr_train_tc_kernel.cuh"
@@ -222,7 +224,8 @@ __global__ void flmr_simt_maxsim_kernel(const __nv_bfloat16* __restrict__ d, con
 // reference packs each bucket index LSB-first into big-endian bytes: residual.py:188-204 binarize,
 // :51-73 reversed_bit_map, :77-93 lookup table; decode loop decompress_residuals.cpp:27-78), then the
 // row is L2-normalised (index_storage.py:173) and stored as bf16.  HBM-bound byte work: one warp per
-// token, lane = 4 dims, centroid rows come from L2, bucket weights from shared memory.
+// token, lane = 4 dims, centroid rows come from L2, bucket weights from shared memory.  The arithmetic is
+// flmr_scan_plaid_kernel.cuh's plaid_* functions, so a compressed corpus decodes to the same bits.
 __global__ void flmr_plaid_decode_kernel(const int32_t* __restrict__ codes,
                                          const uint8_t* __restrict__ residuals,
                                          const float* __restrict__ centroids,
@@ -235,9 +238,7 @@ __global__ void flmr_plaid_decode_kernel(const int32_t* __restrict__ codes,
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
-  const int keys = 8 / nbits;                 // bucket indices per packed byte
   const int packed_dim = kDim * nbits / 8;    // bytes per token
-  const uint32_t mask = (1u << nbits) - 1u;
   for (int64_t t = warp0; t < n_tokens; t += n_warps) {
     const int32_t code = codes[t];
     if (code < 0 || code >= n_centroids) {    // corrupt index: flag, never read out of bounds
@@ -249,19 +250,10 @@ __global__ void flmr_plaid_decode_kernel(const int32_t* __restrict__ codes,
     }
     const float4 c = __ldg(reinterpret_cast<const float4*>(centroids + static_cast<int64_t>(code) * kDim) + lane);
     const uint8_t* row = residuals + t * packed_dim;
-    float v[4] = {c.x, c.y, c.z, c.w};
-#pragma unroll
-    for (int dd = 0; dd < 4; ++dd) {
-      const int i = 4 * lane + dd;
-      const uint32_t byte = __ldg(row + i / keys);
-      const uint32_t field = (byte >> (8 - nbits * (i % keys + 1))) & mask;
-      v[dd] += s_w[__brev(field) >> (32 - nbits)];
-    }
+    float v[4];
+    plaid_lane_values(c, row, s_w, nbits, lane, v);
     if (normalize) {
-      float ss = v[0] * v[0] + v[1] * v[1] + v[2] * v[2] + v[3] * v[3];
-#pragma unroll
-      for (int off = 16; off >= 1; off >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, off);
-      const float inv = 1.0f / fmaxf(sqrtf(ss), 1e-12f);   // torch.nn.functional.normalize eps
+      const float inv = plaid_inv_norm(v);
 #pragma unroll
       for (int dd = 0; dd < 4; ++dd) v[dd] *= inv;
     }
@@ -529,6 +521,15 @@ struct flmr_corpus {
   uint32_t* d_pair_end_mask = nullptr;
   int32_t* d_pair_first_pid = nullptr;
   CUtensorMap tmap_half;
+  // compressed (PLAID) residency, flmr_corpus_create_plaid: nbits != 0 and d_tokens == nullptr.  Rows in the
+  // padded order above plus kTileN zero rows; the scan decodes them (flmr_scan_plaid_kernel.cuh)
+  int nbits = 0;
+  int64_t n_centroids = 0;
+  int32_t* d_codes = nullptr;          // [n_rows + kTileN]
+  uint8_t* d_residuals = nullptr;      // [n_rows + kTileN][16 * nbits]
+  float* d_inv_norm = nullptr;         // [n_rows + kTileN]
+  float* d_centroids = nullptr;        // [n_centroids][128]
+  float* d_weights = nullptr;          // [2^nbits]
 };
 
 // Streaming corpus construction (index load): the padded token matrix is allocated once, packed rows arrive in
@@ -549,6 +550,20 @@ struct flmr_corpus_builder {
   int64_t *d_soff = nullptr, *d_poff = nullptr;
   int next = 0;
   double fill_s = 0.0;                  // host time spent filling the pinned buffers (read / memcpy)
+};
+
+// Chunked construction of a compressed corpus (flmr_corpus_plaid_builder_*): the handle's arrays are allocated once
+// from the doclens, then chunks of whole passages are packed into them in order, so a load holds no more than the
+// resident arrays plus the caller's current chunk.
+struct flmr_corpus_plaid_builder {
+  flmr_corpus* corpus = nullptr;        // under construction (owned until finish)
+  std::vector<int64_t> soff, poff;
+  std::vector<int32_t> doclens;
+  int64_t passages_done = 0;
+  int sm_count = 0;
+  cudaStream_t stream = nullptr;
+  int64_t *d_soff = nullptr, *d_poff = nullptr;
+  int* d_bad = nullptr;                 // set by the pack kernel when a code is out of range
 };
 
 struct flmr_workspace {
@@ -649,6 +664,19 @@ int dev_upload(T** dptr, const std::vector<T>& h, int64_t* bytes_acc) {
   FLMR_CUDA(cudaMalloc(reinterpret_cast<void**>(dptr), bytes));
   if (!h.empty()) FLMR_CUDA(cudaMemcpy(*dptr, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice));
   if (bytes_acc) *bytes_acc += static_cast<int64_t>(bytes);
+  return FLMR_OK;
+}
+
+// FLMR_OK if every pointer is device memory of `device` (or managed).
+int check_device_ptrs(std::initializer_list<const void*> ptrs, int device) {
+  for (const void* ptr : ptrs) {
+    cudaPointerAttributes attr{};
+    const bool ok = cudaPointerGetAttributes(&attr, ptr) == cudaSuccess &&
+                    ((attr.type == cudaMemoryTypeDevice && attr.device == device) ||
+                     attr.type == cudaMemoryTypeManaged);
+    cudaGetLastError();
+    if (!ok) return fail(FLMR_ERR_INVALID_ARG, "PLAID arrays must be device pointers on device %d", device);
+  }
   return FLMR_OK;
 }
 
@@ -801,7 +829,17 @@ int launch_scan(const flmr_corpus* c, flmr_workspace* ws, ScanParams p, bool pai
     FLMR_CUDA(cudaEventRecord(ev.a, st));
   }
   (void)ws;
-  if (pair) {
+  if (c->nbits) {
+    // compressed corpus: the decoding kernel, single-CTA passes on the two-warpgroup structure (never planned as
+    // pairs: n_pairs = 0), whatever the scan variant
+    const PlaidParams q{c->d_codes, c->d_residuals, c->d_inv_norm, c->d_centroids, c->d_weights};
+    switch (c->nbits) {
+      case 1: flmr_scan_plaid_kernel<1><<<c->n_ctas, kPlaidThreads, PlaidSmem<1>::kBytes, st>>>(p, q); break;
+      case 2: flmr_scan_plaid_kernel<2><<<c->n_ctas, kPlaidThreads, PlaidSmem<2>::kBytes, st>>>(p, q); break;
+      case 4: flmr_scan_plaid_kernel<4><<<c->n_ctas, kPlaidThreads, PlaidSmem<4>::kBytes, st>>>(p, q); break;
+      default: flmr_scan_plaid_kernel<8><<<c->n_ctas, kPlaidThreads, PlaidSmem<8>::kBytes, st>>>(p, q); break;
+    }
+  } else if (pair) {
     // clusters of two CTAs share one of the n_pairs token ranges; the tensor map has a half-tile box
     p.cta_row_begin = c->d_pair_row_begin;
     p.cta_tile_base = c->d_pair_tile_base;
@@ -1021,6 +1059,23 @@ int finish_corpus(flmr_corpus* c, const std::vector<int64_t>& poff, const int32_
     if ((rc = dev_upload(&c->d_tile_end_mask, end_mask, &c->hbm_bytes))) return bail(rc);
     if ((rc = dev_upload(&c->d_tile_first_pid, first_pid, &c->hbm_bytes))) return bail(rc);
   }
+  if (c->nbits) {   // compressed: no tensor map, no CTA-pair partition; the decoding kernel's smem attribute
+    cudaError_t e = cudaFuncSetAttribute(flmr_scan_plaid_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         PlaidSmem<1>::kBytes);
+    if (e == cudaSuccess)
+      e = cudaFuncSetAttribute(flmr_scan_plaid_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               PlaidSmem<2>::kBytes);
+    if (e == cudaSuccess)
+      e = cudaFuncSetAttribute(flmr_scan_plaid_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               PlaidSmem<4>::kBytes);
+    if (e == cudaSuccess)
+      e = cudaFuncSetAttribute(flmr_scan_plaid_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               PlaidSmem<8>::kBytes);
+    if (e != cudaSuccess)
+      return bail(fail(FLMR_ERR_CUDA, "cannot raise the dynamic shared memory limit of the compressed scan: %s",
+                       cudaGetErrorString(e)));
+    return FLMR_OK;
+  }
   if ((rc = encode_rows_map(&c->tmap_d, c->d_tokens, static_cast<uint64_t>(n_rows), kTileN)))
     return bail(rc);
   if (n_ctas >= 2 && n_passages >= n_ctas / 2) {   // CTA-pair experiment: its own partition + half-tile tensor map
@@ -1191,6 +1246,176 @@ int flmr_corpus_create(const void* tokens, const int32_t* h_doclens, int64_t n_p
   return FLMR_OK;
 }
 
+int flmr_corpus_plaid_builder_create(const float* d_centroids, int64_t n_centroids, const float* d_bucket_weights,
+                                     int nbits, const int32_t* h_doclens, int64_t n_passages, int dim, int device,
+                                     int64_t pid_base, flmr_corpus_plaid_builder_t** out) {
+  if (!out) return fail(FLMR_ERR_INVALID_ARG, "out is null");
+  *out = nullptr;
+  if (dim != kDim) return fail(FLMR_ERR_UNSUPPORTED, "dim=%d (only %d is supported)", dim, kDim);
+  if (nbits != 1 && nbits != 2 && nbits != 4 && nbits != 8)
+    return fail(FLMR_ERR_INVALID_ARG, "nbits=%d (the PLAID codec packs 1, 2, 4 or 8 bits per dim)", nbits);
+  if (!d_centroids || !d_bucket_weights || !h_doclens) return fail(FLMR_ERR_INVALID_ARG, "null pointer");
+  if (n_passages <= 0 || n_centroids < 1)
+    return fail(FLMR_ERR_INVALID_ARG, "bad sizes n_passages=%lld n_centroids=%lld", (long long)n_passages,
+                (long long)n_centroids);
+  flmr_corpus_plaid_builder* b = new (std::nothrow) flmr_corpus_plaid_builder();
+  if (!b) return fail(FLMR_ERR_OOM, "host allocation failed");
+  auto bail = [&](int code) {
+    flmr_corpus_plaid_builder_destroy(b);
+    return code;
+  };
+  b->soff.resize(n_passages + 1);
+  b->poff.resize(n_passages + 1);
+  b->doclens.assign(h_doclens, h_doclens + n_passages);
+  b->soff[0] = b->poff[0] = 0;
+  for (int64_t p = 0; p < n_passages; ++p) {
+    const int32_t len = h_doclens[p];
+    if (len < 1)
+      return bail(fail(FLMR_ERR_INVALID_ARG,
+                       "passage %lld has length %d; zero-length passages have no defined MaxSim score",
+                       (long long)p, len));
+    b->soff[p + 1] = b->soff[p] + len;
+    b->poff[p + 1] = b->poff[p] + (static_cast<int64_t>(len) + kGroup - 1) / kGroup * kGroup;
+  }
+  const int64_t n_rows = b->poff[n_passages];
+  if (n_rows + kTileN >= (1ll << 31))
+    return bail(fail(FLMR_ERR_UNSUPPORTED,
+                     "%lld stored token rows exceed the 2^31 per-shard limit; shard the corpus", (long long)n_rows));
+  DeviceGuard guard(device);
+  if (!guard.ok) return bail(fail(FLMR_ERR_CUDA, "cudaSetDevice(%d) failed", device));
+  cudaDeviceProp prop;
+  cudaError_t e = cudaGetDeviceProperties(&prop, device);
+  if (e != cudaSuccess) return bail(fail(FLMR_ERR_CUDA, "cudaGetDeviceProperties: %s", cudaGetErrorString(e)));
+  if (prop.major != 10)
+    return bail(fail(FLMR_ERR_UNSUPPORTED, "device %d is sm_%d%d; this library is sm_100a only", device, prop.major,
+                     prop.minor));
+  b->sm_count = prop.multiProcessorCount;
+  if (int rc = check_device_ptrs({d_centroids, d_bucket_weights}, device)) return bail(rc);
+
+  flmr_corpus* c = new (std::nothrow) flmr_corpus();
+  if (!c) return bail(fail(FLMR_ERR_OOM, "host allocation failed"));
+  b->corpus = c;
+  c->device = device;
+  c->n_passages = n_passages;
+  c->n_tokens = b->soff[n_passages];
+  c->n_rows = n_rows;
+  c->pid_base = pid_base;
+  c->nbits = nbits;
+  c->n_centroids = n_centroids;
+  const int packed = kDim * nbits / 8;
+  const int64_t rows_alloc = n_rows + kTileN;   // + one tile of zero rows: the last tile never reads past the end
+  auto alloc = [&](void** ptr, size_t bytes) -> int {
+    cudaError_t err = cudaMalloc(ptr, bytes);
+    if (err != cudaSuccess)
+      return fail(FLMR_ERR_OOM, "cudaMalloc(%zu B) for the compressed corpus failed: %s", bytes,
+                  cudaGetErrorString(err));
+    c->hbm_bytes += static_cast<int64_t>(bytes);
+    return FLMR_OK;
+  };
+  int rc;
+  if ((rc = alloc(reinterpret_cast<void**>(&c->d_codes), static_cast<size_t>(rows_alloc) * 4)) ||
+      (rc = alloc(reinterpret_cast<void**>(&c->d_residuals), static_cast<size_t>(rows_alloc) * packed)) ||
+      (rc = alloc(reinterpret_cast<void**>(&c->d_inv_norm), static_cast<size_t>(rows_alloc) * 4)) ||
+      (rc = alloc(reinterpret_cast<void**>(&c->d_centroids), static_cast<size_t>(n_centroids) * kDim * 4)) ||
+      (rc = alloc(reinterpret_cast<void**>(&c->d_weights), static_cast<size_t>(4) << nbits)))
+    return bail(rc);
+  if ((rc = dev_upload(&b->d_soff, b->soff, nullptr)) || (rc = dev_upload(&b->d_poff, b->poff, nullptr)))
+    return bail(rc);
+  if ((e = cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking)) != cudaSuccess ||
+      (e = cudaMalloc(reinterpret_cast<void**>(&b->d_bad), sizeof(int))) != cudaSuccess ||
+      (e = cudaMemsetAsync(b->d_bad, 0, sizeof(int), b->stream)) != cudaSuccess ||
+      (e = cudaMemcpyAsync(c->d_centroids, d_centroids, static_cast<size_t>(n_centroids) * kDim * 4,
+                           cudaMemcpyDeviceToDevice, b->stream)) != cudaSuccess ||
+      (e = cudaMemcpyAsync(c->d_weights, d_bucket_weights, static_cast<size_t>(4) << nbits, cudaMemcpyDeviceToDevice,
+                           b->stream)) != cudaSuccess ||
+      (e = cudaMemsetAsync(c->d_codes + n_rows, 0, kTileN * 4, b->stream)) != cudaSuccess ||
+      (e = cudaMemsetAsync(c->d_residuals + n_rows * packed, 0, static_cast<size_t>(kTileN) * packed, b->stream)) !=
+          cudaSuccess ||
+      (e = cudaMemsetAsync(c->d_inv_norm + n_rows, 0, kTileN * 4, b->stream)) != cudaSuccess ||
+      (e = cudaStreamSynchronize(b->stream)) != cudaSuccess)   // the caller may free the centroids on return
+    return bail(fail(FLMR_ERR_CUDA, "compressed corpus setup: %s", cudaGetErrorString(e)));
+  *out = b;
+  return FLMR_OK;
+}
+
+int flmr_corpus_plaid_builder_append(flmr_corpus_plaid_builder_t* b, const int32_t* d_codes,
+                                     const uint8_t* d_residuals, int64_t n_tokens) {
+  if (!b || !d_codes || !d_residuals) return fail(FLMR_ERR_INVALID_ARG, "null argument");
+  flmr_corpus* c = b->corpus;
+  const int64_t pa = b->passages_done;
+  const int64_t want = b->soff[pa] + n_tokens;
+  const int64_t pb = std::lower_bound(b->soff.begin() + pa, b->soff.end(), want) - b->soff.begin();
+  if (n_tokens <= 0 || pb > c->n_passages || b->soff[pb] != want)
+    return fail(FLMR_ERR_INVALID_ARG,
+                "an append must hold whole passages: %lld tokens after passage %lld do not end on a passage boundary",
+                (long long)n_tokens, (long long)pa);
+  DeviceGuard guard(c->device);
+  if (!guard.ok) return fail(FLMR_ERR_CUDA, "cudaSetDevice(%d) failed", c->device);
+  if (int rc = check_device_ptrs({d_codes, d_residuals}, c->device)) return rc;
+  const int threads = 256;
+  const int64_t cnt = pb - pa;
+  flmr_plaid_pack_kernel<<<static_cast<unsigned>((cnt * 32 + threads - 1) / threads), threads, 0, b->stream>>>(
+      d_codes, d_residuals, b->d_soff, b->d_poff, pa, cnt, b->soff[pa], c->d_centroids, c->n_centroids, c->d_weights,
+      c->nbits, c->d_codes, c->d_residuals, c->d_inv_norm, b->d_bad);
+  ++g_launches;
+  FLMR_CUDA(cudaGetLastError());
+  FLMR_CUDA(cudaStreamSynchronize(b->stream));   // the caller may free or refill the chunk on return
+  b->passages_done = pb;
+  return FLMR_OK;
+}
+
+int flmr_corpus_plaid_builder_finish(flmr_corpus_plaid_builder_t* b, flmr_corpus_t** out) {
+  if (!b || !out) return fail(FLMR_ERR_INVALID_ARG, "null argument");
+  *out = nullptr;
+  flmr_corpus* c = b->corpus;
+  if (b->passages_done != c->n_passages)
+    return fail(FLMR_ERR_INVALID_ARG, "%lld of %lld passages appended", (long long)b->passages_done,
+                (long long)c->n_passages);
+  DeviceGuard guard(c->device);
+  if (!guard.ok) return fail(FLMR_ERR_CUDA, "cudaSetDevice(%d) failed", c->device);
+  int bad = 0;
+  FLMR_CUDA(cudaMemcpyAsync(&bad, b->d_bad, sizeof(int), cudaMemcpyDeviceToHost, b->stream));
+  FLMR_CUDA(cudaStreamSynchronize(b->stream));
+  if (bad) return fail(FLMR_ERR_INVALID_ARG, "a centroid code is outside [0, %lld)", (long long)c->n_centroids);
+  if (int rc = finish_corpus(c, b->poff, b->doclens.data(), b->sm_count)) return rc;
+  b->corpus = nullptr;   // ownership passes to the caller
+  flmr_corpus_plaid_builder_destroy(b);
+  *out = c;
+  return FLMR_OK;
+}
+
+int flmr_corpus_plaid_builder_destroy(flmr_corpus_plaid_builder_t* b) {
+  if (!b) return FLMR_OK;
+  if (b->stream) cudaStreamSynchronize(b->stream);
+  cudaFree(b->d_soff);
+  cudaFree(b->d_poff);
+  cudaFree(b->d_bad);
+  if (b->stream) cudaStreamDestroy(b->stream);
+  if (b->corpus) flmr_corpus_destroy(b->corpus);
+  delete b;
+  return FLMR_OK;
+}
+
+int flmr_corpus_create_plaid(const int32_t* d_codes, const uint8_t* d_residuals, const float* d_centroids,
+                             int64_t n_centroids, const float* d_bucket_weights, int nbits, const int32_t* h_doclens,
+                             int64_t n_passages, int dim, int device, int64_t pid_base, flmr_corpus_t** out) {
+  if (!out) return fail(FLMR_ERR_INVALID_ARG, "out is null");
+  *out = nullptr;
+  if (!d_codes || !d_residuals) return fail(FLMR_ERR_INVALID_ARG, "null pointer");
+  flmr_corpus_plaid_builder_t* b = nullptr;
+  int rc = flmr_corpus_plaid_builder_create(d_centroids, n_centroids, d_bucket_weights, nbits, h_doclens, n_passages,
+                                            dim, device, pid_base, &b);
+  if (rc) return rc;
+  if ((rc = flmr_corpus_plaid_builder_append(b, d_codes, d_residuals, b->soff[n_passages])) ||
+      (rc = flmr_corpus_plaid_builder_finish(b, out))) {
+    const std::string msg = g_last_error;
+    flmr_corpus_plaid_builder_destroy(b);
+    g_last_error = msg;
+    return rc;
+  }
+  return FLMR_OK;
+}
+
 int flmr_corpus_destroy(flmr_corpus_t* c) {
   if (!c) return FLMR_OK;
   DeviceGuard guard(c->device);
@@ -1205,6 +1430,11 @@ int flmr_corpus_destroy(flmr_corpus_t* c) {
   cudaFree(c->d_pair_tile_base);
   cudaFree(c->d_pair_end_mask);
   cudaFree(c->d_pair_first_pid);
+  cudaFree(c->d_codes);
+  cudaFree(c->d_residuals);
+  cudaFree(c->d_inv_norm);
+  cudaFree(c->d_centroids);
+  cudaFree(c->d_weights);
   delete c;
   return FLMR_OK;
 }
@@ -1570,6 +1800,14 @@ int flmr_corpus_gather(const flmr_corpus_t* c, const int64_t* d_pids, int64_t n_
   const int threads = 256;
   const int64_t blocks = (n_pids * nd_max * 32 + threads - 1) / threads;
   if (blocks > 0x7fffffffll) return fail(FLMR_ERR_UNSUPPORTED, "gather of %lld x %d rows is too large", (long long)n_pids, nd_max);
+  if (c->nbits) {   // compressed corpus: decode the gathered rows
+    flmr_gather_plaid_kernel<<<static_cast<unsigned>(blocks), threads, 0, static_cast<cudaStream_t>(stream)>>>(
+        c->d_codes, c->d_residuals, c->d_inv_norm, c->d_centroids, c->d_weights, c->nbits, c->d_poff, c->d_doclen,
+        d_pids, n_pids, nd_max, c->n_passages, c->pid_base, static_cast<uint2*>(d_out_bf16), d_mask);
+    FLMR_CUDA(cudaGetLastError());
+    ++g_launches;
+    return FLMR_OK;
+  }
   flmr_gather_kernel<<<static_cast<unsigned>(blocks), threads, 0, static_cast<cudaStream_t>(stream)>>>(
       reinterpret_cast<const uint2*>(c->d_tokens), c->d_poff, c->d_doclen, d_pids, n_pids, nd_max,
       c->n_passages, c->pid_base, static_cast<uint2*>(d_out_bf16), d_mask);
@@ -1812,6 +2050,7 @@ int flmr_debug_maxsim_scores_simt(const flmr_corpus_t* c, const void* d_q, int n
   if (n_queries <= 0 || nq <= 0) return fail(FLMR_ERR_INVALID_ARG, "bad shape");
   if (c->n_passages > 0x7fffffffll || n_queries > 65535)
     return fail(FLMR_ERR_UNSUPPORTED, "SIMT cross-check grid too large");
+  if (c->nbits) return fail(FLMR_ERR_UNSUPPORTED, "the SIMT cross-check reads bf16 tokens; this corpus is compressed");
   DeviceGuard guard(c->device);
   if (!guard.ok) return fail(FLMR_ERR_CUDA, "cudaSetDevice(%d) failed", c->device);
   const int threads = nq >= 256 ? 256 : (nq > 128 ? 256 : 128);
